@@ -2,6 +2,7 @@
 """bench.py — agent-env-steps/sec of the gather-trade-build step (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -62,6 +63,37 @@ WORKLOADS = {
                     "64 agents, 64x64, 2048 env replicas per GPU",
                l2="no explicit flush: each step rewrites 740 MB of observations (> 126 MB L2) and touches 126 MB of state"),
 }
+
+
+# what a caller of the step receives, per workload family (the stepper's output buffers)
+GTB_OUTPUTS = ["obs_agent_map", "obs_agent_idx", "obs_agent_flat", "mask_agent", "obs_planner_map", "obs_planner_idx",
+               "obs_planner_flat", "obs_planner_agents", "mask_planner", "obs_time", "reward", "done"]
+COVID_OUTPUTS = ["obs_agent_state", "obs_postsubsidy", "obs_lagged_stringency", "obs_policy_indicators", "obs_scalars",
+                 "mask_agent", "mask_planner", "reward_agent", "reward_planner", "done"]
+DUMP_BYTES = 60 * 10 ** 6   # under 64 MB with the .npy headers
+
+
+def sample_outputs(bufs, names, E):
+    """--dump-outputs: the step's output buffers for a fixed, seeded sample of env replicas (all of them when they fit in
+    DUMP_BYTES), copied to the host as float32, or float64 where float32 would not hold every value (f64, i32), and the
+    sampled replicas' indices as env_index."""
+    import torch
+
+    ts = {n: bufs[n] for n in names if n in bufs}
+    wide = {n for n, t in ts.items() if t.dtype in (torch.float64, torch.int32, torch.int64)}
+    per_env = 8 + sum(t[0].numel() * (8 if n in wide else 4) for n, t in ts.items())   # 8: env_index
+    n_env = int(min(E, DUMP_BYTES // max(1, per_env)))
+    rows = np.sort(np.random.RandomState(0).choice(E, n_env, replace=False))
+    idx = torch.as_tensor(rows, device=next(iter(ts.values())).device)
+    out = {n: t.index_select(0, idx).to("cpu", torch.float64 if n in wide else torch.float32).numpy() for n, t in ts.items()}
+    out["env_index"] = rows.astype(np.float64)
+    return out
+
+
+def write_outputs(outdir, arrays):
+    os.makedirs(outdir, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(outdir, n + ".npy"), a)
 
 
 def workload_config(key, E):
@@ -385,7 +417,7 @@ class Ctx:
         return float(np.median(per)), len(per), float(min(per)), float(max(per))
 
 
-def measure_gtb(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20, e2e_mode="compact", e2e_threads=0):
+def measure_gtb(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20, e2e_mode="compact", e2e_threads=0, dump=False):
     """One gather-trade-build workload on this rank's GPU: value / sustained / per-kernel roofline / e2e."""
     import ctypes as C
 
@@ -432,6 +464,7 @@ def measure_gtb(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20, e2e_mode="c
         clocks.mark_begin()
     ms_total = ctx.time_steps(one_step, K)
     launches = st.launch_count() - launches0
+    outputs = sample_outputs(st.buf, GTB_OUTPUTS, E) if dump else None
     sus_ms, sus_n, sus_min, sus_max = ctx.sustained(one_step, K, ms_total)
     if clocks:
         clocks.mark_end()
@@ -493,8 +526,7 @@ def measure_gtb(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20, e2e_mode="c
 
     # ---- e2e through the host entry point with pinned HOST buffers ----
     out_host, out_ptrs, d2h = {}, {}, 0
-    for nm in ["obs_agent_map", "obs_agent_idx", "obs_agent_flat", "mask_agent", "obs_planner_map", "obs_planner_idx",
-               "obs_planner_flat", "obs_planner_agents", "mask_planner", "obs_time", "reward", "done"]:
+    for nm in GTB_OUTPUTS:
         if nm in st.buf:
             # pinned host tensors from the package's allocator: blocks of replicas (one transfer slice each) on alternating
             # NUMA nodes, which is what the node-pinned expansion threads of aie_step_host_compact are matched to: every
@@ -560,7 +592,7 @@ def measure_gtb(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20, e2e_mode="c
         "config": dict(workload_config(key, E), parallelism="env replicas sharded over %d GPU(s), no collective on "
                        "the step path" % world, setup_s=t_setup, device_reset=("reference-exact (reset_mode 1)"
                        if env.spec.get("reset_mode", 0) == 1 else "snapshot restore (reset_mode 0)")),
-        "e2e": e2e, "gpu_launches": launches, "roofline": roofline, "dtype": "i32+f64", "n_agents": A,
+        "e2e": e2e, "gpu_launches": launches, "roofline": roofline, "dtype": "i32+f64", "n_agents": A, "outputs": outputs,
     }
     if with_cpu:
         res["cpu_baseline"] = cpu_baseline_for(key)
@@ -590,7 +622,7 @@ def measure_gtb(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20, e2e_mode="c
     return res
 
 
-def measure_covid(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20):
+def measure_covid(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20, dump=False):
     """BASELINE config 4: one fused kernel per step (+ the random-policy sampler)."""
     torch, args, rank, world, dev = ctx.torch, ctx.args, ctx.rank, ctx.world, ctx.dev
     from ai_economist_b200 import foundation
@@ -616,6 +648,7 @@ def measure_covid(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20):
         clocks.mark_begin()
     ms_total = ctx.time_steps(one_step, K)
     launches = st.launch_count() - l0
+    outputs = sample_outputs(st.buf, COVID_OUTPUTS, E) if dump else None
     sus_ms, sus_n, sus_min, sus_max = ctx.sustained(one_step, K, ms_total, max_repeats=20)
     if clocks:
         clocks.mark_end()
@@ -645,8 +678,7 @@ def measure_covid(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20):
     dom = "aie_covid_step_kernel"
     traffic, traffic_src = committed_traffic(key, dom)
     # e2e: pinned host actions in, all outputs back
-    names = ["obs_agent_state", "obs_postsubsidy", "obs_lagged_stringency", "obs_policy_indicators", "obs_scalars",
-             "mask_agent", "mask_planner", "reward_agent", "reward_planner", "done"]
+    names = COVID_OUTPUTS
     host = {n: torch.empty(st.buf[n].shape, dtype=st.buf[n].dtype, pin_memory=True) for n in names}
     act_a = torch.zeros((E, S), dtype=torch.int32, pin_memory=True)
     act_p = torch.zeros((E,), dtype=torch.int32, pin_memory=True)
@@ -679,7 +711,7 @@ def measure_covid(ctx, key, K, W, with_cpu, clocks=None, e2e_steps=20):
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": E * (S + 1) * 4, "d2h_bytes_per_step": d2h,
                 "steps": n_e2e, "what": "pinned host actions -> device, step, every observation/mask/reward/done tensor "
                                         "back to pinned host"},
-        "gpu_launches": launches, "dtype": "f32+f64", "n_agents": S,
+        "gpu_launches": launches, "dtype": "f32+f64", "n_agents": S, "outputs": outputs,
         "roofline": {"bound": "hbm", "kernel": dom, "achieved": kernels[dom]["achieved_gbs"], "peak": peak, "unit": "GB/s",
                      "frac": kernels[dom]["frac"], "traffic": traffic, "traffic_source": traffic_src,
                      "peak_source": peak_src, "alg_bytes_per_env_step": step_bytes, "kernels": kernels},
@@ -762,6 +794,9 @@ def main():
     ap.add_argument("--preroll", type=int, default=None, help="untimed steps after staggering the episode phases (default: one episode)")
     ap.add_argument("--no-extra-workloads", action="store_true",
                     help="headline workload only (skip the c3/c4/c5 entries of `workloads`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (a fixed, seeded sample of env replicas "
+                         "when the whole batch exceeds 64 MB; rank 0's replicas)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -791,7 +826,9 @@ def main():
         # 2 x 32-core B200 host and burn half the CPU time, profiles/r02z_e2e_transfer_knobs.txt section 7)
         args.e2e_threads = max(8, host_cores() // (2 * max(1, world)))
     kw = {} if key == "c4" else dict(e2e_mode=args.e2e_mode, e2e_threads=args.e2e_threads)
-    res = fn(ctx, key, args.steps, args.warmup, with_cpu, clocks=clocks, e2e_steps=args.e2e_steps, **kw)
+    res = fn(ctx, key, args.steps, args.warmup, with_cpu, clocks=clocks, e2e_steps=args.e2e_steps,
+             dump=bool(args.dump_outputs) and rank == 0, **kw)
+    outputs = res.pop("outputs")
     clk = clocks.stop() if clocks else None
     extra = {}
     if key == "c2" and not args.no_extra_workloads and not args.envs_per_gpu:
@@ -820,6 +857,8 @@ def main():
         line["vs_reference_cuda"] = res["vs_reference_cuda"]
     if extra:
         line["workloads"] = extra
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

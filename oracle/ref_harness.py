@@ -1,8 +1,9 @@
 """TEST INFRASTRUCTURE ONLY — imports the *unmodified* reference from /root/reference.
 
 Used (a) to validate the C restatement in oracle/ and (b) to generate the golden
-fixtures committed under tests/golden/.  /root/reference does not exist on the GPU
-box, so nothing under `-m gpu`, smoke() or bench.py may import this module.
+fixtures committed under tests/golden/ (including the recorded digests of
+oracle/ref_tape.py).  The reference is not part of the repository, so nothing under
+`-m gpu`, smoke() or bench.py may load it (load_reference_foundation).
 
 Recipe follows SURVEY.md Appendix C: stub the absent third-party modules the
 reference imports at module scope (lz4, Crypto, GPUtil), restore `np.int`.
@@ -258,3 +259,11 @@ def sample_actions(env, obs, rng):
             off += d
         actions["p"] = p_row
     return actions, np.array(a_rows, np.int32), np.array(p_row, np.int32)
+
+
+def sample_actions_from_masks(env, a_mask, p_mask, rng):
+    """sample_actions on masks held as arrays (a_mask [A, L], p_mask [L]) with the agents of a product env: the same
+    draws as sample_actions on the reference's observation wherever the masks are equal."""
+    obs = {str(i): {"action_mask": np.asarray(a_mask[i])} for i in range(env.n_agents)}
+    obs["p"] = {"action_mask": np.asarray(p_mask).reshape(-1)}
+    return sample_actions(env, obs, rng)

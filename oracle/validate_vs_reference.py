@@ -10,23 +10,9 @@ import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import ref_harness as rh  # noqa: E402
+from oracle import ref_tape  # noqa: E402
 from oracle.oracle import OracleBatch  # noqa: E402
 from oracle.configs import CONFIGS  # noqa: E402
-
-
-def compare(name, a, b, exact=True, rtol=1e-6, atol=1e-9):
-    a, b = np.asarray(a), np.asarray(b)
-    if a.shape != b.shape:
-        return "%s: shape %s vs %s" % (name, a.shape, b.shape)
-    if exact:
-        if not np.array_equal(a, b):
-            idx = np.argwhere(a != b)[:5]
-            return "%s: mismatch at %s ref=%s orc=%s" % (name, idx.tolist(), a[tuple(idx[0])], b[tuple(idx[0])])
-    else:
-        if not np.allclose(a, b, rtol=rtol, atol=atol):
-            idx = np.argwhere(~np.isclose(a, b, rtol=rtol, atol=atol))[:5]
-            return "%s: mismatch at %s ref=%s orc=%s" % (name, idx.tolist(), a[tuple(idx[0])], b[tuple(idx[0])])
-    return None
 
 
 EXACT_STATE = ["cell", "owner", "loc", "inv", "esc", "n_orders", "bid_hist", "ask_hist", "tax_pos", "rate_idx",
@@ -36,57 +22,77 @@ EXACT_OBS = ["a_map", "a_idx", "a_mask", "p_map", "p_idx", "p_mask", "done"]
 CLOSE_OBS = ["a_flat", "p_flat", "p_agents", "time", "rew"]
 
 
-def run(cfg_name, seed, steps, verbose=True):
-    f = rh.load_reference_foundation()
-    cfg = dict(CONFIGS[cfg_name])
-    env = f.make_env_instance(**cfg)
+def product_env(cfg, seed):
+    """The product's host-side reset of a reference configuration (spec and post-reset state for the oracle)."""
+    from ai_economist_b200 import foundation
+    kw = dict(cfg)
+    name = kw.pop("scenario_name")
+    env = foundation.make_env_instance(name, n_envs=1, stepper_factory=lambda *a, **k: None, auto_reset=False, seed=None, **kw)
     env.seed(seed)
-    obs = env.reset()
-    spec = rh.spec_from_reference_env(env)
+    return env, {k: v[0] for k, v in env.host_reset_arrays().items()}
+
+
+RESET_KEYS = ["stone", "wood", "stone_src", "wood_src", "water", "loc", "mt_key", "mt_pos", "coin", "build_payment",
+              "build_skill", "bonus_gather_prob"]
+
+
+def run(cfg_name, seed, steps, verbose=True, tape=None):
+    """The C oracle against the reference, step by step.  tape (oracle/ref_tape.py): None compares with the live reference;
+    a replaying tape compares with its recorded digests, the oracle then starting from the product's host-side reset
+    (which recording checks against the reference's post-reset state) and drawing the same actions from its own masks."""
+    tape = tape or ref_tape.Tape()
+    cfg = dict(CONFIGS[cfg_name])
+    prod, host = product_env(cfg, seed)
+    if tape.live:
+        f = rh.load_reference_foundation()
+        env = f.make_env_instance(**cfg)
+        env.seed(seed)
+        obs = env.reset()
+        spec = rh.spec_from_reference_env(env)
+        state = rh.state_from_reference_env(env)
+    else:
+        spec, state = prod.spec, host
+    if tape.live and not set(spec) <= set(prod.spec):
+        raise RuntimeError("spec keys the product lacks: %s" % sorted(set(spec) - set(prod.spec)))
+    for k in tape.keys("spec", [k for k in sorted(prod.spec) if k != "components"], spec if tape.live else ()):
+        tape.equal("spec/" + k, spec[k] if tape.live else None, prod.spec[k])
+    for k in RESET_KEYS:
+        tape.equal("reset/" + k, state[k] if tape.live else None, host[k])
     orc = OracleBatch(spec, 1)
-    orc.load_env(0, rh.state_from_reference_env(env))
+    orc.load_env(0, state)
     arng = np.random.RandomState(seed + 7919)
-    errs = []
 
-    def check(t, obs, rew=None, done=None):
-        ro = rh.obs_arrays_from_reference(env, obs, rew, done)
+    def check(t, obs=None, rew=None, done=None):
+        ro = rs = {}
+        if tape.live:
+            ro = rh.obs_arrays_from_reference(env, obs, rew, done)
+            rs = rh.state_arrays_from_reference(env)
         oo = orc.obs(0)
-        rs = rh.state_arrays_from_reference(env)
         os_ = orc.state(0)
-        for k in EXACT_OBS:
-            if k in ro:
-                e = compare(k, ro[k], oo[k]); errs.append(e) if e else None
-        for k in CLOSE_OBS:
-            if k in ro:
-                e = compare(k, ro[k], oo[k], exact=False, rtol=1e-6, atol=1e-7); errs.append(e) if e else None
-        for k in EXACT_STATE:
-            if k in rs:
-                e = compare(k, rs[k], os_[k]); errs.append(e) if e else None
-        for k in CLOSE_STATE:
-            if k in rs:
-                e = compare(k, rs[k], os_[k], exact=False, rtol=1e-9, atol=1e-9); errs.append(e) if e else None
-        if "book" in rs:
-            for (c, side), rows in rs["book"].items():
-                e = compare("book%d%d" % (c, side), rows, orc.book(0, c, side)); errs.append(e) if e else None
-        if errs:
-            print("[%s seed %d] step %d: %d mismatches" % (cfg_name, seed, t, len(errs)))
-            for e in errs[:10]:
-                print("   ", e)
-            return False
-        return True
+        where = "[%s seed %d] step %d:" % (cfg_name, seed, t)
+        for k in tape.keys("exact_obs%d" % bool(t), EXACT_OBS, ro):
+            tape.equal(k, ro.get(k), oo[k], where, shape=True)
+        for k in tape.keys("close_obs%d" % bool(t), CLOSE_OBS, ro):
+            tape.close(k, ro.get(k), oo[k], rtol=1e-6, atol=1e-7, where=where, shape=True)
+        for k in tape.keys("exact_state", EXACT_STATE, rs):
+            tape.equal(k, rs.get(k), os_[k], where, shape=True)
+        for k in tape.keys("close_state", CLOSE_STATE, rs):
+            tape.close(k, rs.get(k), os_[k], rtol=1e-9, atol=1e-9, where=where, shape=True)
+        for c, side in tape.keys("book", [(0, 0), (0, 1), (1, 0), (1, 1)], rs.get("book", {})):
+            tape.equal("book%d%d" % (c, side), rs["book"][(c, side)] if tape.live else None, orc.book(0, c, side), where, shape=True)
 
-    if not check(0, obs):
-        return False
-    n_trades = n_builds = 0
+    check(0, obs if tape.live else None)
     for t in range(1, steps + 1):
-        actions, a_act, p_act = rh.sample_actions(env, obs, arng)
-        obs, rew, done, _ = env.step(actions)
+        o = orc.obs(0)
+        actions, a_act, p_act = rh.sample_actions_from_masks(prod, o["a_mask"], o["p_mask"], arng)
+        if tape.live:
+            obs, rew, done, _ = env.step(actions)
         orc.step(a_act[None], p_act[None] if p_act.size else None)
-        if not check(t, obs, rew, done):
-            return False
-        if done["__all__"]:
+        check(t, *((obs, rew, done) if tape.live else ()))
+        if int(orc.obs(0)["done"][0]):
             break
-    if verbose:
+    tape.finish()
+    if verbose and tape.live:
         m = env.metrics
         print("[%s seed %d] %d steps OK  (trades=%s, builds=%s)" % (
             cfg_name, seed, t, m.get("Trade/n_trades", m.get("ContinuousDoubleAuction/n_trades")),
@@ -103,5 +109,9 @@ if __name__ == "__main__":
     ok = True
     for c in a.configs:
         for s in [int(x) for x in a.seeds.split(",")]:
-            ok &= run(c, s, a.steps)
+            try:
+                run(c, s, a.steps)
+            except ref_tape.Mismatch as ex:
+                print("[%s seed %d] %s" % (c, s, ex))
+                ok = False
     sys.exit(0 if ok else 1)

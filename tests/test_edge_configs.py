@@ -2,7 +2,7 @@
 order slot, 32 price levels, no auction / no build component, tax every step, disabled taxes, linear / log brackets,
 eta near 1, unscaled observations, a non-square world with 33 agents.
 
-  * build container (reference present): the C oracle and the product's host-side reset against the live reference;
+  * the C oracle and the product's host-side reset against the reference (its recorded values, oracle/ref_tape.py);
   * everywhere: the device source (1-lane emulation) against the oracle through the public API;
   * `-m gpu`: the CUDA build against the oracle, same harness (ordered last, see tests/conftest.py).
 """
@@ -11,6 +11,7 @@ import pytest
 
 from oracle import configs
 from oracle import ref_harness as rh
+from oracle import ref_tape
 
 EDGE = sorted(configs.EDGE_CONFIGS)
 
@@ -46,29 +47,31 @@ def test_emulated_device_code_matches_oracle_on_edge_config(cfg):
     run_against_oracle(make_product_env(cfg, 3, emu_factory, seed=900), steps=40, check_every=10)
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rh.reference_available(), reason="reference tree not present")
 @pytest.mark.parametrize("cfg", EDGE)
 def test_oracle_and_host_reset_track_live_reference_on_edge_config(cfg):
     from oracle.validate_vs_reference import run
     _all_configs()
-    assert run(cfg, 501, 40, verbose=False)
+    assert run(cfg, 501, 40, verbose=False, tape=ref_tape.Tape("edge_oracle", cfg))
     # the product's host-side reset: same spec, same post-reset state, same stream position
-    f = rh.load_reference_foundation()
-    ref = f.make_env_instance(**configs.EDGE_CONFIGS[cfg])
-    ref.seed(77)
-    ref.reset()
-    want_spec, want = rh.spec_from_reference_env(ref), rh.state_from_reference_env(ref)
+    tape = ref_tape.Tape("edge_host_reset", cfg)
+    want_spec = want = {}
+    if tape.live:
+        f = rh.load_reference_foundation()
+        ref = f.make_env_instance(**configs.EDGE_CONFIGS[cfg])
+        ref.seed(77)
+        ref.reset()
+        want_spec, want = rh.spec_from_reference_env(ref), rh.state_from_reference_env(ref)
     env = make_product_env(cfg, 1, lambda *a, **k: None, seed=None)
     env.seed(77)
     got = env.host_reset_arrays()
-    for k, v in want_spec.items():
-        if k != "components":
-            assert env.spec[k] == v, k
+    assert set(want_spec) <= set(env.spec), sorted(set(want_spec) - set(env.spec))
+    for k in tape.keys("spec", [k for k in sorted(env.spec) if k != "components"], want_spec):
+        tape.equal(k, want_spec.get(k), env.spec[k])
     for k in ["stone", "wood", "stone_src", "wood_src", "water", "loc", "mt_key", "coin", "build_payment",
               "build_skill", "bonus_gather_prob"]:
-        assert np.array_equal(np.asarray(got[k][0]), np.asarray(want[k])), k
-    assert int(got["mt_pos"][0]) == int(want["mt_pos"])
+        tape.equal(k, want.get(k), np.asarray(got[k][0]))
+    tape.equal("mt_pos", int(want["mt_pos"]) if tape.live else None, int(got["mt_pos"][0]))
+    tape.finish()
 
 
 @pytest.mark.gpu

@@ -7,15 +7,17 @@ profiles/); here every fuzzer contributes N_CASES configurations drawn from a fi
 
   * emu vs oracle            CPU, always            the device source (1-lane emulation) against the C oracle
   * cuda vs oracle           -m gpu                 the same configurations on the CUDA build (through the C-ABI)
-  * oracle vs reference      -m reference           the C oracle against the live imported reference
-  * device reset vs ref.     -m reference           reference-exact auto-reset across 4 episodes against env.reset()
-  * reference API vs ref.    -m reference           ReferenceApiEnv against the reference: obs, rewards, metrics, dense logs
-  * dynamic layouts vs ref.  -m reference           uniform / quadrant: device-side layout generation at every auto-reset
-  * one-step-economy vs ref. -m reference           SimpleLabor + one-step-economy incl. finished-episode metrics
-  * Saez hybrid vs reference -m reference           the Saez tax model (device / host), with and without tax annealing
-  * COVID vs reference       -m reference           COVID device code (scan and change list) under parameter variants
+  * oracle vs reference      CPU, always            the C oracle against the reference
+  * device reset vs ref.     CPU, always            reference-exact auto-reset across 4 episodes against env.reset()
+  * reference API vs ref.    CPU, always            ReferenceApiEnv against the reference: obs, rewards, metrics, dense logs
+  * dynamic layouts vs ref.  CPU, always            uniform / quadrant: device-side layout generation at every auto-reset
+  * one-step-economy vs ref. CPU, always            SimpleLabor + one-step-economy incl. finished-episode metrics
+  * Saez hybrid vs reference CPU, always            the Saez tax model (device / host), with and without tax annealing
+  * COVID vs reference       CPU, always            COVID device code (scan and change list) under parameter variants
 
-`-m reference` cases need /root/reference (build container) and are skipped elsewhere.
+The cases against the reference compare with its values as recorded from the unmodified reference
+(tests/golden/reference_tapes/, oracle/ref_tape.py; AIE_RECORD_REFERENCE=1 records them again where the reference is
+importable).  A case whose configuration the reference itself refused when it was recorded is skipped.
 """
 import os
 import sys
@@ -27,15 +29,25 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 import fuzz_emu_vs_oracle as fz  # noqa: E402
-from oracle import ref_harness as rh  # noqa: E402
+from oracle import ref_tape  # noqa: E402
 
 N_CASES = 20
-needs_reference = pytest.mark.skipif(not rh.reference_available(), reason="reference tree not present")
 
 
 def _configs(seed, n=N_CASES, draw=None):
     rng = np.random.RandomState(seed)
     return [(draw or fz.random_config)(rng) for _ in range(n)]
+
+
+def _against_reference(family, case, fn, refusals=(), when=lambda ex: True):
+    """fn(tape) against the recorded reference (the live one while recording); `refusals`: exceptions by which the
+    reference refuses a configuration (recorded; the case is then skipped)."""
+    try:
+        tape = ref_tape.Tape(family, case)
+        with tape.refusals(refusals, when):
+            fn(tape)
+    except ref_tape.Refused as ex:
+        pytest.skip("the reference refused the configuration: %s" % ex)
 
 
 def _skip_unsupported(fn, *a, **k):
@@ -77,8 +89,6 @@ def test_fuzz_cuda_matches_oracle(i):
     bu.run_pair(env, orc, min(60, kw["episode_length"]), np.random.RandomState(1 + i), check_every=15)
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(N_CASES))
 def test_fuzz_oracle_matches_live_reference(i):
     from oracle import configs
@@ -86,25 +96,18 @@ def test_fuzz_oracle_matches_live_reference(i):
 
     name, kw = _configs(5)[i]
     configs.CONFIGS["_fuzz"] = dict(kw, scenario_name=name)
-    try:
-        ok = run("_fuzz", 100 + i, min(60, kw["episode_length"]), verbose=False)
-    except (AssertionError, NotImplementedError, TimeoutError) as ex:   # the reference refusing its own configuration
-        pytest.skip("reference / harness refused the configuration: %r" % (ex,))
-    assert ok
+    _against_reference("fuzz_oracle", i, lambda tape: run("_fuzz", 100 + i, min(60, kw["episode_length"]), verbose=False, tape=tape),
+                       (AssertionError, NotImplementedError, TimeoutError))   # the reference refusing its own configuration
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(N_CASES))
 def test_fuzz_device_reset_matches_live_reference(i):
     import fuzz_device_reset_vs_reference as fr
 
     cfg = _configs(0, draw=fr.random_config)[i]
-    fr.run_one(cfg, seed=500 + i, episodes=3)
+    _against_reference("fuzz_device_reset", i, lambda tape: fr.run_one(cfg, seed=500 + i, episodes=3, tape=tape))
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(N_CASES))
 def test_fuzz_dynamic_layout_device_reset_matches_live_reference(i):
     """uniform / quadrant: the device generates a new clumped layout at every auto-reset (rand thinning, randn + convolve2d
@@ -112,14 +115,10 @@ def test_fuzz_dynamic_layout_device_reset_matches_live_reference(i):
     import fuzz_device_reset_vs_reference as fr
 
     cfg = _configs(11, draw=fr.random_dynamic_config)[i]
-    try:
-        fr.run_one(cfg, seed=600 + i, episodes=3)
-    except TimeoutError as ex:   # the reference's own placement loop giving up on a crowded map
-        pytest.skip(repr(ex))
+    _against_reference("fuzz_dynamic_layout", i, lambda tape: fr.run_one(cfg, seed=600 + i, episodes=3, tape=tape),
+                       (TimeoutError,))   # the reference's own placement loop giving up on a crowded map
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(10))
 def test_fuzz_multi_zone_device_reset_matches_live_reference(i, monkeypatch):
     """multi_zone: np.random.shuffle of the region -> zone-type vector on the device before every layout."""
@@ -127,16 +126,12 @@ def test_fuzz_multi_zone_device_reset_matches_live_reference(i, monkeypatch):
 
     monkeypatch.setattr(fr, "FAMILIES", ["multi_zone"])
     cfg = _configs(21, n=10, draw=fr.random_dynamic_config)[i]
-    try:
-        fr.run_one(cfg, seed=650 + i, episodes=3)
-    except (TimeoutError, AssertionError) as ex:
-        if isinstance(ex, AssertionError) and "coverage" not in str(ex) and "World" not in str(ex):
-            raise
-        pytest.skip(repr(ex))   # the reference refusing its own configuration
+    # the reference refusing its own configuration: placement timeouts, its coverage / world asserts
+    _against_reference("fuzz_multi_zone", i, lambda tape: fr.run_one(cfg, seed=650 + i, episodes=3, tape=tape),
+                       (TimeoutError, AssertionError),
+                       lambda ex: not isinstance(ex, AssertionError) or "coverage" in str(ex) or "World" in str(ex))
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(10))
 def test_fuzz_saez_hybrid_matches_live_reference(i):
     """PeriodicBracketTax(tax_model="saez"): warm-up draws on the device, buffer / regression / formula on the host, rates in
@@ -145,21 +140,18 @@ def test_fuzz_saez_hybrid_matches_live_reference(i):
     import fuzz_device_reset_vs_reference as fr
 
     cfg = _configs(31, n=10, draw=fr.random_saez_config)[i]
-    fr.run_one(cfg, seed=800 + i, episodes=fr.saez_episodes(cfg))
+    _against_reference("fuzz_saez", i, lambda tape: fr.run_one(cfg, seed=800 + i, episodes=fr.saez_episodes(cfg), tape=tape))
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(N_CASES))
 def test_fuzz_reference_api_matches_live_reference(i):
     import fuzz_reference_api_vs_reference as fa
 
     name, kw = _configs(0)[i]
-    _skip_unsupported(fa.run_one, name, kw, seed=700 + i)
+    _against_reference("fuzz_reference_api", i, lambda tape: fa.run_one(name, kw, seed=700 + i, tape=tape),
+                       (NotImplementedError, TimeoutError))   # unsupported / unbuildable configurations
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(N_CASES))
 def test_fuzz_one_step_economy_matches_live_reference(i):
     """SimpleLabor + one-step-economy (components/simple_labor.py, scenarios/one_step_economy): observations, masks, rewards,
@@ -167,14 +159,12 @@ def test_fuzz_one_step_economy_matches_live_reference(i):
     import fuzz_one_step_vs_reference as fo
 
     cfg = _configs(3, draw=fo.random_config)[i]
-    fo.run_one(cfg, seed=300 + i, episodes=3)
+    _against_reference("fuzz_one_step_economy", i, lambda tape: fo.run_one(cfg, seed=300 + i, episodes=3, tape=tape))
 
 
-@needs_reference
-@pytest.mark.reference
 @pytest.mark.parametrize("i", range(8))
 def test_fuzz_covid_matches_live_reference(i):
     import fuzz_covid_vs_reference as fc
 
     kw = _configs(0, n=8, draw=fc.random_kwargs)[i]
-    fc.run_one(kw, 900 + i)
+    _against_reference("fuzz_covid", i, lambda tape: fc.run_one(kw, 900 + i, tape=tape))

@@ -89,46 +89,44 @@ def test_one_step_economy_rejects_what_the_reference_rejects():
         foundation.make_env_instance("one-step-economy", components=[("SimpleLabor", {})], labor_exponent=1.0, **base)
 
 
-@pytest.mark.reference
 def test_reference_api_facade_runs_the_one_step_economy_like_the_reference():
     """reference_api=True: the reference's single-env interface (nested dicts, named fields) over replica 0, side by side with
-    the live reference through three episodes: observations, rewards, done, metrics."""
+    the reference through three episodes: observations, rewards, done, metrics (the reference's values as recorded,
+    oracle/ref_tape.py)."""
     from oracle import ref_harness as rh
-    if not rh.reference_available():
-        pytest.skip("reference tree not present")
+    from oracle import ref_tape
+    from oracle.ref_tape import same_metrics, same_tree
     from tests.emu.emu_stepper import emu_factory
     cfg = dict(components=[("SimpleLabor", dict(mask_first_step=True, payment_max_skill_multiplier=3)),
                            ("PeriodicBracketTax", dict(bracket_spacing="us-federal", period=2, tax_model="model_wrapper", rate_disc=0.05))],
                n_agents=6, world_size=[1, 1], episode_length=2, flatten_observations=False, flatten_masks=True)
     env = foundation.make_env_instance("one-step-economy", reference_api=True, stepper_factory=emu_factory, seed=5, **cfg)
     env.seed(7)
-    f = rh.load_reference_foundation()
-    np.random.seed(5)
-    ref = f.make_env_instance(scenario_name="one-step-economy", **cfg)
-    ref.seed(7)
-
-    def same(a, b, label):
-        assert set(a) == set(b), (label, sorted(set(a) ^ set(b)))
-        for k in a:
-            if isinstance(a[k], dict):
-                same(a[k], b[k], label + "/" + k)
-            else:
-                assert np.allclose(np.asarray(a[k], float), np.asarray(b[k], float), rtol=1e-6, atol=1e-7), label + "/" + k
+    tape = ref_tape.Tape("one_step_economy_facade", 0)
+    if tape.live:
+        f = rh.load_reference_foundation()
+        np.random.seed(5)
+        ref = f.make_env_instance(scenario_name="one-step-economy", **cfg)
+        ref.seed(7)
 
     rng = np.random.RandomState(1)
+    o1 = r1 = d1 = m1 = None
     for ep in range(3):
-        o1, o2 = ref.reset(), env.reset()
-        same(o1, o2, "ep %d reset" % ep)
+        if tape.live:
+            o1 = ref.reset()
+        o2 = env.reset()
+        same_tree(tape, "obs", o1, o2, "ep %d reset" % ep)
         for t in range(2):
-            acts = {str(i): int(rng.choice(np.flatnonzero(np.asarray(o1[str(i)]["action_mask"])))) for i in range(6)}
-            pm = np.asarray(o1["p"]["action_mask"]).reshape(7, -1)
+            acts = {str(i): int(rng.choice(np.flatnonzero(np.asarray(o2[str(i)]["action_mask"])))) for i in range(6)}
+            pm = np.asarray(o2["p"]["action_mask"]).reshape(7, -1)
             acts["p"] = [int(rng.choice(np.flatnonzero(pm[b]))) for b in range(7)]
-            (o1, r1, d1, _), (o2, r2, d2, _) = ref.step(acts), env.step(acts)
-            same(o1, o2, "ep %d t %d obs" % (ep, t)); same(r1, r2, "ep %d t %d rew" % (ep, t))
-            assert d1 == d2
+            if tape.live:
+                o1, r1, d1, _ = ref.step(acts)
+            o2, r2, d2, _ = env.step(acts)
+            same_tree(tape, "obs", o1, o2, "ep %d t %d obs" % (ep, t))
+            same_tree(tape, "rew", r1, r2, "ep %d t %d rew" % (ep, t))
+            tape.equal("done", ref_tape.flags(d1) if tape.live else None, ref_tape.flags(d2), "ep %d t %d" % (ep, t))
         with np.errstate(all="ignore"):
-            m1, m2 = ref.metrics, env.metrics
-        assert set(m1) == set(m2)
-        for k, v in m1.items():
-            a, b = float(v), float(m2[k])
-            assert (np.isnan(a) and np.isnan(b)) or abs(a - b) <= 1e-6 * max(1.0, abs(a)), k
+            m1 = ref.metrics if tape.live else None
+            same_metrics(tape, "metrics", m1, env.metrics, "ep %d" % ep)
+    tape.finish()

@@ -6,6 +6,8 @@ import pytest
 
 from ai_economist_b200 import foundation
 from oracle import ref_harness as rh
+from oracle import ref_tape
+from oracle.ref_tape import same_tree
 from tests.emu.emu_stepper import emu_factory
 
 # tutorials/economic_simulation_basic.ipynb cell 11, verbatim apart from a shorter episode
@@ -69,46 +71,56 @@ def test_tutorial_loop_runs_unchanged_on_the_reference_api():
     assert m is not None and "social/productivity" in m
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rh.reference_available(), reason="reference tree not present")
 @pytest.mark.parametrize("flags", [dict(flatten_observations=False, flatten_masks=True),
                                    dict(flatten_observations=True, flatten_masks=True),
                                    # schedules that live across resets: the "auto" warm-up integrator, completions
                                    dict(energy_warmup_constant=3, energy_warmup_method="auto", episode_length=30),
                                    dict(energy_warmup_constant=2, energy_warmup_method="decay", episode_length=30)],
                          ids=["named_fields", "flat", "auto_warmup", "decay_warmup"])
-def test_reference_api_tracks_the_live_reference(flags):
-    """Same config, same seed, same caller code on both: identical observation structure and values, two episodes."""
+def test_reference_api_tracks_the_live_reference(flags, request):
+    """Same config, same seed, same caller code on both: identical observation structure and values, two episodes (the
+    reference's values as recorded, oracle/ref_tape.py)."""
     cfg = dict(ENV_CONFIG)
     cfg.update(flags)
-    f = rh.load_reference_foundation()
-    ref = f.make_env_instance(**cfg)
+    tape = ref_tape.Tape("reference_api", request.node.callspec.id)
+    if tape.live:
+        f = rh.load_reference_foundation()
+        ref = f.make_env_instance(**cfg)
     mine = foundation.make_env_instance(**cfg, reference_api=True, stepper_factory=emu_factory)
-    ref.seed(9)
+    if tape.live:
+        ref.seed(9)
     mine.seed(9)
 
-    def same(a, b, label):
-        if isinstance(a, dict):
-            assert set(a.keys()) == set(b.keys()), label
-            for k in a:
-                same(a[k], b[k], label + "/" + str(k))
+    def leaf_types(b, label):
+        if isinstance(b, dict):
+            for k in b:
+                leaf_types(b[k], label + "/" + str(k))
         else:
             assert type(b) in (float, list, np.ndarray, bool), (label, type(b))
-            assert np.allclose(np.asarray(a, np.float64), np.asarray(b, np.float64), rtol=1e-6, atol=1e-7), label
 
+    o1 = r1 = d1 = None
     for episode in range(3):
         ra, rb = np.random.RandomState(episode), np.random.RandomState(episode)
-        o1, o2 = ref.reset(), mine.reset()
-        same(o1, o2, "reset %d" % episode)
-        for t in range(ref.episode_length):
-            a1, a2 = sample_random_actions(ref, o1, ra), sample_random_actions(mine, o2, rb)
-            assert {k: int(v) for k, v in a1.items() if k != "p"} == {k: int(v) for k, v in a2.items() if k != "p"}
-            (o1, r1, d1, _), (o2, r2, d2, _) = ref.step(a1), mine.step(a2)
-            same(o1, o2, "ep %d t %d obs" % (episode, t))
-            same(r1, r2, "ep %d t %d rew" % (episode, t))
-            assert d1 == d2
-    mref, mmine = ref.metrics, mine.metrics
-    assert set(mref) == set(mmine)
+        if tape.live:
+            o1 = ref.reset()
+        o2 = mine.reset()
+        leaf_types(o2, "reset %d" % episode)
+        same_tree(tape, "obs", o1, o2, "reset %d" % episode)
+        for t in range(mine.episode_length):
+            a2 = sample_random_actions(mine, o2, rb)
+            if tape.live:
+                a1 = sample_random_actions(ref, o1, ra)
+            agents = sorted(k for k in a2 if k != "p")
+            tape.equal("actions", [int(a1[k]) for k in agents] if tape.live else None, [int(a2[k]) for k in agents], "ep %d t %d" % (episode, t))
+            if tape.live:
+                o1, r1, d1, _ = ref.step(a1)
+            o2, r2, d2, _ = mine.step(a2)
+            leaf_types(o2, "ep %d t %d obs" % (episode, t)); leaf_types(r2, "ep %d t %d rew" % (episode, t))
+            same_tree(tape, "obs", o1, o2, "ep %d t %d obs" % (episode, t))
+            same_tree(tape, "rew", r1, r2, "ep %d t %d rew" % (episode, t))
+            tape.equal("done", ref_tape.flags(d1) if tape.live else None, ref_tape.flags(d2), "ep %d t %d" % (episode, t))
+    tape.equal("metric keys", sorted(ref.metrics) if tape.live else None, sorted(mine.metrics))
+    tape.finish()
 
 
 @pytest.mark.gpu
@@ -167,36 +179,57 @@ def test_replay_log_reproduces_an_episode():
     assert env.previous_episode_dense_log["Trade"] == want_log["Trade"]
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rh.reference_available(), reason="reference tree not present")
+def _log_text(log):
+    """A replay log as canonical text (numpy scalars and arrays as numbers and lists)."""
+    import json
+    return json.dumps(log, sort_keys=True, default=lambda o: o.tolist() if hasattr(o, "tolist") else str(o))
+
+
 def test_a_replay_log_recorded_by_the_reference_replays_here():
     """Cross-implementation replay: the unmodified reference plays an episode and hands over its replay log; replaying
-    that log through the facade ends in the reference's final state and metrics (and the other way round)."""
-    f = rh.load_reference_foundation()
-    ref = f.make_env_instance(**ENV_CONFIG)
-    ref.seed(5)
-    play(ref, np.random.RandomState(3), dense=False)
-    log = ref.previous_episode_replay_log
-    want = rh.state_arrays_from_reference(ref)
+    that log through the facade ends in the reference's final state and metrics (and the other way round).  The
+    reference's log, end states and metrics are the ones recorded from it (oracle/ref_tape.py); the log the facade
+    writes for the same play must be the reference's."""
+    tape = ref_tape.Tape("reference_api_replay_log", 0)
+    here = foundation.make_env_instance(**ENV_CONFIG, reference_api=True, stepper_factory=emu_factory)
+    here.seed(5)
+    play(here, np.random.RandomState(3), dense=False)
+    log = here.previous_episode_replay_log
+    want = {}
+    if tape.live:
+        f = rh.load_reference_foundation()
+        ref = f.make_env_instance(**ENV_CONFIG)
+        ref.seed(5)
+        play(ref, np.random.RandomState(3), dense=False)
+        tape.equal("log", _log_text(ref.previous_episode_replay_log), _log_text(log))
+        log = ref.previous_episode_replay_log
+        want = rh.state_arrays_from_reference(ref)
+    else:
+        tape.equal("log", None, _log_text(log))
     mine = foundation.make_env_instance(**ENV_CONFIG, reference_api=True, stepper_factory=emu_factory)
     mine.reset(**log["reset"])
     for s in log["step"]:
         mine.step(**s)
     got = _final_state(mine)
     for k in ["cell", "owner", "loc", "inv", "esc", "mt_key"]:
-        assert np.array_equal(np.asarray(want[k]), got[k].reshape(np.asarray(want[k]).shape)), k
-    assert np.allclose(want["coin"], got["coin"], rtol=1e-9) and np.allclose(want["labor"], got["labor"], rtol=1e-9)
-    m_ref, m_mine = ref.metrics, mine.metrics
-    assert set(m_ref) == set(m_mine)
-    for k, v in m_ref.items():
-        assert np.isclose(float(v), float(m_mine[k]), rtol=1e-6, atol=1e-9, equal_nan=True), k
+        tape.equal(k, want.get(k), got[k])
+    tape.close("coin", want.get("coin"), got["coin"], rtol=1e-9, atol=1e-8)
+    tape.close("labor", want.get("labor"), got["labor"], rtol=1e-9, atol=1e-8)
+    m_mine = mine.metrics
+    m_ref = ref.metrics if tape.live else {}
+    tape.equal("metric keys", sorted(m_ref) if tape.live else None, sorted(m_mine))
+    for k in sorted(m_mine):
+        tape.close("metric/" + k, m_ref.get(k), float(m_mine[k]), rtol=1e-6, atol=1e-9, equal_nan=True)
     # ... and a log recorded here drives the reference to the same end state
     mine.seed(8)
     play(mine, np.random.RandomState(4), dense=False)
     log2, want2 = mine.previous_episode_replay_log, _final_state(mine)
-    ref.reset(**log2["reset"])
-    for s in log2["step"]:
-        ref.step(**s)
-    got2 = rh.state_arrays_from_reference(ref)
+    got2 = {}
+    if tape.live:
+        ref.reset(**log2["reset"])
+        for s in log2["step"]:
+            ref.step(**s)
+        got2 = rh.state_arrays_from_reference(ref)
     for k in ["cell", "owner", "loc", "inv", "esc", "mt_key"]:
-        assert np.array_equal(np.asarray(got2[k]), want2[k].reshape(np.asarray(got2[k]).shape)), k
+        tape.equal("replayed/" + k, got2.get(k), want2[k])
+    tape.finish()

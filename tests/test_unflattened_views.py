@@ -5,6 +5,7 @@ import pytest
 
 from ai_economist_b200 import foundation
 from oracle import ref_harness as rh
+from oracle import ref_tape
 from oracle.configs import CONFIGS
 from tests.emu.emu_stepper import emu_factory
 
@@ -47,47 +48,51 @@ def test_named_fields_are_slices_of_the_flat_vectors(cfg):
     assert total + n_noop == np.asarray(flat.obs["0"]["action_mask"]).shape[-1]
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rh.reference_available(), reason="reference tree not present")
 @pytest.mark.parametrize("cfg", ["c1_tutorial", "c3_short_period", "tax_us_federal", "full_obs_tax"])
 def test_unflattened_observations_match_live_reference(cfg):
-    f = rh.load_reference_foundation()
-    kw = dict(CONFIGS[cfg])
-    kw.update(flatten_observations=False, flatten_masks=False)
-    ref = f.make_env_instance(**kw)
-    ref.seed(21)
-    ref_obs = ref.reset()
+    """The named fields and per-subspace masks against the reference's (its values as recorded, oracle/ref_tape.py)."""
+    tape = ref_tape.Tape("unflattened_views", cfg)
+    ref_obs = None
+    if tape.live:
+        f = rh.load_reference_foundation()
+        kw = dict(CONFIGS[cfg])
+        kw.update(flatten_observations=False, flatten_masks=False)
+        ref = f.make_env_instance(**kw)
+        ref.seed(21)
+        ref_obs = ref.reset()
     env = _product(cfg, flatten_observations=False, flatten_masks=False)
     env.seed([21, 22])
     obs = env.reset()
     rng = np.random.RandomState(4)
 
-    def compare(ro, po, label):
-        assert set(ro.keys()) == set(po.keys()), "%s: %s" % (label, sorted(set(ro) ^ set(po)))
-        for k, rv in ro.items():
-            if isinstance(rv, dict):
-                compare(rv, po[k], label + "/" + k)
+    def compare(ro, po, key, label):
+        tape.equal(key + "/", sorted(ro) if tape.live else None, sorted(po), label)
+        for k in sorted(po):
+            if isinstance(po[k], dict) or (tape.live and isinstance(ro[k], dict)):
+                compare(ro[k] if tape.live else None, po[k], key + "/" + k, label)
                 continue
             got = np.asarray(po[k])[0]
-            want = np.asarray(rv, dtype=np.float64).reshape(got.shape)
-            assert np.allclose(want, got, rtol=1e-6, atol=1e-7), "%s/%s ref=%s got=%s" % (label, k, want, got)
+            want = np.asarray(ro[k], dtype=np.float64).reshape(got.shape) if tape.live else None
+            tape.close(key + "/" + k, want, got, rtol=1e-6, atol=1e-7, where=label)
 
     for t in range(25):
-        for idx in ref_obs:
-            compare(ref_obs[idx], obs[idx], "t=%d agent %s" % (t, idx))
+        tape.equal("agents", sorted(ref_obs) if tape.live else None, sorted(obs), "t=%d" % t)
+        for idx in sorted(obs):
+            compare(ref_obs[idx] if tape.live else None, obs[idx], idx, "t=%d agent %s" % (t, idx))
         actions, a_act, p_act = {}, [], None
-        for i in range(ref.n_agents):          # a random unmasked action per agent, from the reference's mask dict
-            ag = ref.get_agent(i)
+        for i in range(env.n_agents):          # a random unmasked action per agent, from the mask dict
+            ag = env.get_agent(i)
+            mask = {n: np.asarray(obs[str(i)]["action_mask"][n], float)[0] for n in ag._action_names}
             if ag.multi_action_mode:
-                row = [int(rng.choice(len(m) + 1, p=np.r_[1, m] / (1 + np.sum(m))))
-                       for m in (np.asarray(ref_obs[str(i)]["action_mask"][n], float) for n in ag._action_names)]
+                row = [int(rng.choice(len(m) + 1, p=np.r_[1, m] / (1 + np.sum(m)))) for m in (mask[n] for n in ag._action_names)]
                 actions[str(i)] = row
             else:
-                flat_m = np.r_[1.0, np.concatenate([np.asarray(ref_obs[str(i)]["action_mask"][n], float)
-                                                   for n in ag._action_names])]
+                flat_m = np.r_[1.0, np.concatenate([mask[n] for n in ag._action_names])]
                 row = [int(rng.choice(len(flat_m), p=flat_m / flat_m.sum()))]
                 actions[str(i)] = row[0]
             a_act.append(row)
-        ref_obs, _, _, _ = ref.step(actions)
+        if tape.live:
+            ref_obs, _, _, _ = ref.step(actions)
         aa = np.asarray(a_act, np.int32)[None].repeat(2, axis=0)
         obs, _, _, _ = env.step((aa, None))
+    tape.finish()

@@ -14,6 +14,7 @@ sys.path.insert(0, ROOT)
 from ai_economist_b200.foundation.covid19 import build_covid_params  # noqa: E402
 from oracle import gen_golden_covid as gg  # noqa: E402
 from oracle import ref_harness as rh  # noqa: E402
+from oracle import ref_tape  # noqa: E402
 from tests.emu.emu_stepper import EmuCovidStepper  # noqa: E402
 
 KEYS = ["agent_state", "postsubsidy", "lagged", "policy_ind", "scalars", "mask_a", "mask_p"]
@@ -32,11 +33,15 @@ def random_kwargs(rng):
     return kw
 
 
-def run_one(kw, seed):
-    f = rh.load_reference_foundation()
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref = f.make_env_instance(**gg.reference_config(kw))
-        obs = ref.reset()
+def run_one(kw, seed, tape=None):
+    """tape (oracle/ref_tape.py): None compares with the live reference, a replaying tape with its recorded digests.
+    The actions are drawn from the emulation's masks (equal to the reference's, which every check compares)."""
+    tape = tape or ref_tape.Tape()
+    if tape.live:
+        f = rh.load_reference_foundation()
+        with contextlib.redirect_stdout(io.StringIO()):
+            ref = f.make_env_instance(**gg.reference_config(kw))
+            obs = ref.reset()
     p = build_covid_params(**kw)
     emus = [EmuCovidStepper(p, 1, auto_reset=False, change_list=cl) for cl in (False, True)]
     for s in emus:
@@ -51,25 +56,31 @@ def run_one(kw, seed):
     rew_tol, rew_atol = (1e-6, 1e-9) if kw["economic_reward_crra_eta"] == 2.0 else (1e-5, 1e-6)
 
     def check(t, ra):
+        ra = ra or {}
         for s in emus:
             o = s.read_obs(0)
+            where = "t=%d (change_list=%s)" % (t, s.change_list)
             for k in KEYS:
-                assert np.allclose(ra[k], o[k], rtol=1e-6, atol=1e-9), "t=%d %s (change_list=%s)" % (t, k, s.change_list)
+                tape.close(k, ra.get(k), o[k], rtol=1e-6, atol=1e-9, where=where)
             if t:
-                assert np.allclose(ra["rew_a"], o["rew_a"], rtol=rew_tol, atol=rew_atol), "t=%d rew_a (change_list=%s)" % (t, s.change_list)
-                assert np.isclose(float(ra["rew_p"]), float(o["rew_p"]), rtol=rew_tol, atol=rew_atol) and int(ra["done"]) == int(o["done"])
+                tape.close("rew_a", ra.get("rew_a"), o["rew_a"], rtol=rew_tol, atol=rew_atol, where=where)
+                tape.close("rew_p", ra.get("rew_p"), float(o["rew_p"]), rtol=rew_tol, atol=rew_atol, where=where)
+                tape.equal("done", int(ra["done"]) if tape.live else None, int(o["done"]), where)
 
-    check(0, gg.ref_arrays(ref, obs))
+    check(0, gg.ref_arrays(ref, obs) if tape.live else None)
     for t in range(1, kw["episode_length"] + 1):
-        act_a, act_p = gg.sample(obs, rng)
+        o = emus[0].read_obs(0)
+        act_a, act_p = gg.sample({"a": {"action_mask": o["mask_a"]}, "p": {"action_mask": o["mask_p"]}}, rng)
         actions = {str(i): int(act_a[i]) for i in range(51)}
         actions["p"] = int(act_p)
-        obs, rew, done, _ = ref.step(actions)
+        if tape.live:
+            obs, rew, done, _ = ref.step(actions)
         for s in emus:
             s.buf["actions_agent"][0] = act_a
             s.buf["actions_planner"][0] = act_p
             s.step()
-        check(t, gg.ref_arrays(ref, obs, rew, done))
+        check(t, gg.ref_arrays(ref, obs, rew, done) if tape.live else None)
+    tape.finish()
 
 
 if __name__ == "__main__":

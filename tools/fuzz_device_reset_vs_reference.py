@@ -15,6 +15,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from ai_economist_b200 import foundation  # noqa: E402
 from oracle import ref_harness as rh  # noqa: E402
+from oracle import ref_tape  # noqa: E402
 from tests.emu.emu_stepper import emu_factory  # noqa: E402
 
 LAYOUTS = {(15, 15): "env-pure_and_mixed-15x15.txt", (25, 25): "quadrant_25x25_20each_30clump.txt",
@@ -107,11 +108,15 @@ def saez_episodes(cfg):
     return -(-500 // per_episode) + 2
 
 
-def run_one(cfg, seed, episodes=4):
-    f = rh.load_reference_foundation()
-    ref = f.make_env_instance(**cfg)
-    ref.seed(seed)
-    obs = ref.reset()
+def run_one(cfg, seed, episodes=4, tape=None):
+    """tape (oracle/ref_tape.py): None compares with the live reference, a replaying tape with its recorded digests.
+    The actions are drawn from the product's masks (equal to the reference's, which every check compares)."""
+    tape = tape or ref_tape.Tape()
+    if tape.live:
+        f = rh.load_reference_foundation()
+        ref = f.make_env_instance(**cfg)
+        ref.seed(seed)
+        obs = ref.reset()
     kw = dict(cfg)
     name = kw.pop("scenario_name")
     if "seed" in kw:
@@ -125,36 +130,40 @@ def run_one(cfg, seed, episodes=4):
     T = cfg["episode_length"]
 
     def compare(label):
-        ro = rh.obs_arrays_from_reference(ref, obs)
-        rs = rh.state_arrays_from_reference(ref)
+        ro = rs = {}
+        if tape.live:
+            ro = rh.obs_arrays_from_reference(ref, obs)
+            rs = rh.state_arrays_from_reference(ref)
         po, ps = s.read_obs(1), s.read_state(1)
-        for k in ["cell", "owner", "loc", "inv", "esc", "mt_key", "mt_pos", "n_orders"]:
-            if k in rs:
-                assert np.array_equal(rs[k], np.asarray(ps[k]).reshape(np.asarray(rs[k]).shape)), "%s: state %s" % (label, k)
+        for k in tape.keys("state", ["cell", "owner", "loc", "inv", "esc", "mt_key", "mt_pos", "n_orders"], rs):
+            tape.equal(k, rs.get(k), ps[k], label + ": state")
         for k in ["coin", "labor"]:
-            assert np.allclose(rs[k], ps[k], rtol=1e-9, atol=1e-9), "%s: state %s" % (label, k)
+            tape.close(k, rs.get(k), ps[k], rtol=1e-9, atol=1e-9, where=label + ": state")
         for k in ["a_map", "a_idx", "a_mask", "p_mask"]:
-            assert np.array_equal(ro[k], np.asarray(po[k]).reshape(ro[k].shape)), "%s: obs %s" % (label, k)
+            tape.equal(k, ro.get(k), po[k], label + ": obs")
         for k in ["a_flat", "p_flat", "p_agents"]:
-            assert np.allclose(ro[k], np.asarray(po[k]).reshape(ro[k].shape), rtol=1e-6, atol=1e-7), "%s: obs %s" % (label, k)
+            tape.close(k, ro.get(k), po[k], rtol=1e-6, atol=1e-7, where=label + ": obs")
 
     compare("reset")
     for t in range(1, episodes * T + 1):
-        actions, a_act, p_act = rh.sample_actions(ref, obs, arng)
-        obs, rew, done, _ = ref.step(actions)
+        po = s.read_obs(1)
+        actions, a_act, p_act = rh.sample_actions_from_masks(env, po["a_mask"], po["p_mask"], arng)
+        if tape.live:
+            obs, rew, done, _ = ref.step(actions)
         env.step((np.repeat(a_act[None], 2, axis=0), np.repeat(p_act[None], 2, axis=0) if p_act.size else None))
         got_rew = s.to_numpy(s.buf["reward"])[1]
-        want_rew = np.array([rew[str(i)] for i in range(ref.n_agents)] + [rew["p"]])
-        assert np.allclose(want_rew, got_rew, rtol=1e-6, atol=1e-9), "t=%d rewards" % t
-        if done["__all__"]:
-            obs = ref.reset()
+        want_rew = np.array([rew[str(i)] for i in range(ref.n_agents)] + [rew["p"]]) if tape.live else None
+        tape.close("rew", want_rew, got_rew, rtol=1e-6, atol=1e-9, where="t=%d rewards" % t)
+        ended = bool(int(s.to_numpy(s.buf["done"])[1]))
+        tape.equal("done", bool(done["__all__"]) if tape.live else None, ended, "t=%d" % t)
+        if ended:
+            if tape.live:
+                obs = ref.reset()
             with np.errstate(all="ignore"):   # the finished episode's metrics: _finalize_logs vs the device's end-of-episode snapshot
-                p1, p2 = ref.previous_episode_metrics, env.previous_episode_metrics_of(1)
-            assert set(p1) == set(p2), "t=%d previous metrics keys %s" % (t, sorted(set(p1) ^ set(p2))[:5])
-            for k, v in p1.items():
-                a, b = float(v), float(p2[k])
-                assert (np.isnan(a) and np.isnan(b)) or abs(a - b) <= 1e-6 * max(1.0, abs(a)), "t=%d previous metric %s: %r vs %r" % (t, k, a, b)
-        compare("t=%d%s" % (t, " (after reset)" if done["__all__"] else ""))
+                p1 = ref.previous_episode_metrics if tape.live else None
+                ref_tape.same_metrics(tape, "previous metrics", p1, env.previous_episode_metrics_of(1), "t=%d" % t)
+        compare("t=%d%s" % (t, " (after reset)" if ended else ""))
+    tape.finish()
 
 
 if __name__ == "__main__":

@@ -11,6 +11,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from ai_economist_b200 import foundation  # noqa: E402
 from oracle import ref_harness as rh  # noqa: E402
+from oracle import ref_tape  # noqa: E402
 from tests.emu.emu_stepper import emu_factory  # noqa: E402
 
 
@@ -52,54 +53,58 @@ def reference_arrays(ref, obs):
     return out
 
 
-def compare(want, s, e, label):
+def compare(tape, want, s, e, label):
     o, st = s.read_obs(e), s.read_state(e)
+    want = want or {}
     for k in ("a_mask", "p_mask"):
-        assert np.array_equal(want[k], np.asarray(o[k]).reshape(want[k].shape)), "%s: %s" % (label, k)
+        tape.equal(k, want.get(k), o[k], label)
     for k in ("a_flat", "p_flat", "p_agents", "time"):
-        assert np.allclose(want[k], np.asarray(o[k]).reshape(want[k].shape), rtol=1e-6, atol=1e-7), "%s: %s" % (label, k)
-    assert np.array_equal(want["mt_key"], st["mt_key"]) and want["mt_pos"] == int(st["mt_pos"][0]), "%s: numpy stream" % label
+        tape.close(k, want.get(k), o[k], rtol=1e-6, atol=1e-7, where=label)
+    tape.equal("mt_key", want.get("mt_key"), st["mt_key"], label + ": numpy stream")
+    tape.equal("mt_pos", want.get("mt_pos"), int(st["mt_pos"][0]), label + ": numpy stream")
     for k, mine in (("coin", "coin"), ("labor", "labor"), ("production", "build_payment")):
-        assert np.allclose(want[k], st[mine], rtol=1e-9, atol=1e-9), "%s: state %s" % (label, k)
+        tape.close(k, want.get(k), st[mine], rtol=1e-9, atol=1e-9, where=label + ": state")
 
 
-def same_metrics(a, b, label):
-    assert set(a) == set(b), "%s: metric keys %s" % (label, sorted(set(a) ^ set(b))[:6])
-    for k, v in a.items():
-        x, y = float(v), float(b[k])
-        assert (np.isnan(x) and np.isnan(y)) or abs(x - y) <= 1e-6 * max(1.0, abs(x)), "%s: metric %s: %r vs %r" % (label, k, x, y)
-
-
-def run_one(cfg, seed, episodes=4):
-    f = rh.load_reference_foundation()
-    np.random.seed(seed)   # the constructor draws the SimpleLabor skill table from the global stream
-    ref = f.make_env_instance(**cfg)
-    ref.seed(seed + 1)
-    obs = ref.reset()
+def run_one(cfg, seed, episodes=4, tape=None):
+    """tape (oracle/ref_tape.py): None compares with the live reference, a replaying tape with its recorded digests.
+    The actions are drawn from the product's masks (equal to the reference's, which every check compares)."""
+    tape = tape or ref_tape.Tape()
+    if tape.live:
+        f = rh.load_reference_foundation()
+        np.random.seed(seed)   # the constructor draws the SimpleLabor skill table from the global stream
+        ref = f.make_env_instance(**cfg)
+        ref.seed(seed + 1)
+        obs = ref.reset()
     kw = dict(cfg)
     name = kw.pop("scenario_name")
     env = foundation.make_env_instance(name, n_envs=2, stepper_factory=emu_factory, auto_reset=True, seeds=[seed, seed], **kw)
     env.seed([seed + 1, seed + 1])
     env.reset()
     s = env.stepper
-    compare(reference_arrays(ref, obs), s, 1, "reset")
+    compare(tape, reference_arrays(ref, obs) if tape.live else None, s, 1, "reset")
     arng = np.random.RandomState(seed + 2)
-    A, T = ref.n_agents, cfg["episode_length"]
+    A, T = cfg["n_agents"], cfg["episode_length"]
     for t in range(1, episodes * T + 1):
-        actions, a_act, p_act = rh.sample_actions(ref, obs, arng)
-        obs, rew, done, _ = ref.step(actions)
+        po = s.read_obs(1)
+        actions, a_act, p_act = rh.sample_actions_from_masks(env, po["a_mask"], po["p_mask"], arng)
+        if tape.live:
+            obs, rew, done, _ = ref.step(actions)
         env.step((np.repeat(a_act[None], 2, axis=0), np.repeat(p_act[None], 2, axis=0) if p_act.size else None))
-        want_rew = np.array([rew[str(i)] for i in range(A)] + [rew["p"]])
-        got_rew = s.to_numpy(s.buf["reward"])[1]
-        assert np.allclose(want_rew, got_rew, rtol=1e-6, atol=1e-9), "t=%d rewards %s vs %s" % (t, want_rew, got_rew)
-        assert int(done["__all__"]) == int(s.to_numpy(s.buf["done"])[1])
-        if done["__all__"]:
+        want_rew = np.array([rew[str(i)] for i in range(A)] + [rew["p"]]) if tape.live else None
+        tape.close("rew", want_rew, s.to_numpy(s.buf["reward"])[1], rtol=1e-6, atol=1e-9, where="t=%d rewards" % t)
+        ended = bool(int(s.to_numpy(s.buf["done"])[1]))
+        tape.equal("done", bool(done["__all__"]) if tape.live else None, ended, "t=%d" % t)
+        if ended:
+            m_ref = None
+            if tape.live:
+                with np.errstate(all="ignore"):
+                    m_ref = ref.metrics
+                obs = ref.reset()
             with np.errstate(all="ignore"):
-                m_ref = ref.metrics
-            obs = ref.reset()
-            with np.errstate(all="ignore"):
-                same_metrics(m_ref, env.previous_episode_metrics_of(1), "t=%d finished episode" % t)
-        compare(reference_arrays(ref, obs), s, 1, "t=%d" % t)
+                ref_tape.same_metrics(tape, "finished episode", m_ref, env.previous_episode_metrics_of(1), "t=%d" % t)
+        compare(tape, reference_arrays(ref, obs) if tape.live else None, s, 1, "t=%d" % t)
+    tape.finish()
 
 
 if __name__ == "__main__":

@@ -6,6 +6,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tools'))
 import numpy as np
 from oracle import configs
+from oracle import ref_tape
 from oracle.validate_vs_reference import run
 import fuzz_emu_vs_oracle as fz
 rng = np.random.RandomState(int(sys.argv[2]) if len(sys.argv) > 2 else 5)
@@ -16,9 +17,9 @@ for i in range(n):
     cfg = dict(kw, scenario_name=name)
     configs.CONFIGS["_fuzz"] = cfg
     try:
-        ok = run("_fuzz", 100 + i, min(80, kw["episode_length"]), verbose=False)
-        if not ok:
-            bad += 1; print("[%d] MISMATCH %r" % (i, cfg))
+        run("_fuzz", 100 + i, min(80, kw["episode_length"]), verbose=False)
+    except ref_tape.Mismatch as ex:
+        bad += 1; print("[%d] MISMATCH %r\n    %s" % (i, cfg, str(ex)[:300]))
     except Exception as ex:
         msg = "".join(traceback.format_exception_only(type(ex), ex)).strip()[:300]
         print("[%d] exception (reference or harness): %s | %s" % (i, msg, {k: cfg[k] for k in ("scenario_name",)}))

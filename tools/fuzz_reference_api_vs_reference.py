@@ -13,18 +13,8 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 import fuzz_emu_vs_oracle as fz  # noqa: E402
 from ai_economist_b200 import foundation  # noqa: E402
 from oracle import ref_harness as rh  # noqa: E402
+from oracle import ref_tape  # noqa: E402
 from tests.emu.emu_stepper import emu_factory  # noqa: E402
-
-
-def same(a, b, label):
-    if isinstance(a, dict):
-        assert set(a.keys()) == set(b.keys()), "%s keys %s" % (label, sorted(set(a) ^ set(b)))
-        for k in a:
-            same(a[k], b[k], label + "/" + str(k))
-    else:
-        x, y = np.asarray(a, np.float64), np.asarray(b, np.float64)
-        assert x.size == y.size, "%s size %s vs %s" % (label, x.shape, y.shape)
-        assert np.allclose(x.reshape(-1), y.reshape(-1), rtol=1e-6, atol=1e-7), label
 
 
 def pick(env, obs, rng):
@@ -55,42 +45,51 @@ def pick(env, obs, rng):
     return acts
 
 
-def run_one(name, kw, seed):
+def run_one(name, kw, seed, tape=None):
+    """tape (oracle/ref_tape.py): None compares with the live reference, a replaying tape with its recorded digests.
+    The actions are picked from the facade's observations (equal to the reference's, which every check compares)."""
+    import json
+    from oracle.ref_tape import same_log, same_metrics, same_tree
+
+    tape = tape or ref_tape.Tape()
     cfg = dict(kw, scenario_name=name, flatten_observations=bool(seed % 2), flatten_masks=bool((seed // 2) % 2),
                episode_length=12, dense_log_frequency=1, world_dense_log_frequency=5)
-    f = rh.load_reference_foundation()
-    ref = f.make_env_instance(**cfg)
+    if tape.live:
+        f = rh.load_reference_foundation()
+        ref = f.make_env_instance(**cfg)
     mine = foundation.make_env_instance(**cfg, reference_api=True, stepper_factory=emu_factory)
-    ref.seed(seed); mine.seed(seed)
+    if tape.live:
+        ref.seed(seed)
+    mine.seed(seed)
+    o1 = r1 = d1 = p1 = m1 = log1 = None
     for ep in range(3):
         rng = np.random.RandomState(seed * 10 + ep)
-        o1, o2 = ref.reset(), mine.reset()
-        same(o1, o2, "ep %d reset" % ep)
+        if tape.live:
+            o1 = ref.reset()
+        o2 = mine.reset()
+        same_tree(tape, "obs", o1, o2, "ep %d reset" % ep)
         if ep > 0:   # previous_episode_metrics: what _finalize_logs stored when the last episode ended
             with np.errstate(all="ignore"):
-                p1, p2 = ref.previous_episode_metrics, mine.previous_episode_metrics
-            assert set(p1) == set(p2)
-            for k, v in p1.items():
-                a, b = float(v), float(p2[k])
-                assert (np.isnan(a) and np.isnan(b)) or abs(a - b) <= 1e-6 * max(1.0, abs(a)), "ep %d prev metric %s: %r vs %r" % (ep, k, a, b)
+                p1 = ref.previous_episode_metrics if tape.live else None
+                same_metrics(tape, "previous metrics", p1, mine.previous_episode_metrics, "ep %d" % ep)
         for t in range(12):
-            a = pick(ref, o1, rng)
-            (o1, r1, d1, _), (o2, r2, d2, _) = ref.step(a), mine.step(a)
-            same(o1, o2, "ep %d t %d obs" % (ep, t)); same(r1, r2, "ep %d t %d rew" % (ep, t))
-            assert d1 == d2
-        assert int(ref._completions) == mine._completions
+            a = pick(mine, o2, rng)
+            if tape.live:
+                o1, r1, d1, _ = ref.step(a)
+            o2, r2, d2, _ = mine.step(a)
+            same_tree(tape, "obs", o1, o2, "ep %d t %d obs" % (ep, t))
+            same_tree(tape, "rew", r1, r2, "ep %d t %d rew" % (ep, t))
+            tape.equal("done", ref_tape.flags(d1) if tape.live else None, ref_tape.flags(d2), "ep %d t %d" % (ep, t))
+        tape.equal("completions", int(ref._completions) if tape.live else None, mine._completions, "ep %d" % ep)
         # the dense log of the episode that just ended (world / states / actions / rewards + every component's log)
-        from tests.test_dense_log import same as same_log
-        import json
-        same_log(json.loads(json.dumps(ref.previous_episode_dense_log)), json.loads(json.dumps(mine.previous_episode_dense_log)),
-                 "ep %d dense log" % ep)
+        if tape.live:
+            log1 = json.loads(json.dumps(ref.previous_episode_dense_log))
+        same_log(tape, "dense log", log1, json.loads(json.dumps(mine.previous_episode_dense_log)), "ep %d dense log" % ep)
         # env.metrics at the end of the episode (scenario + every component's get_metrics)
         with np.errstate(all="ignore"):
-            m1, m2 = ref.metrics, mine.metrics
-        assert set(m1) == set(m2), "ep %d metrics keys %s" % (ep, sorted(set(m1) ^ set(m2))[:6])
-        for k, v in m1.items():
-            a, b = float(v), float(m2[k])
-            assert (np.isnan(a) and np.isnan(b)) or abs(a - b) <= 1e-6 * max(1.0, abs(a)), "ep %d metric %s: %r vs %r" % (ep, k, a, b)
+            m1 = ref.metrics if tape.live else None
+            same_metrics(tape, "metrics", m1, mine.metrics, "ep %d" % ep)
+    tape.finish()
 
 
 if __name__ == "__main__":
